@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- RANSAC-vote throughput (images*keypoints/s) of the B200-native voting layer.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W]            # our arm (torchrun for N>1)
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]   # our arm (torchrun for N>1)
     python bench.py --impl reference [--gpus N] --steps K --warmup W   # the reference's own path
 
 One "step" = one ransac_voting_layer_v3(mask, vertex, 512, inlier_thresh=0.99) call over one batch of
@@ -224,6 +224,14 @@ def _cpu_baseline(mask, vertex, K, seconds_target=15.0):
                       f"{min(cores, n_img)} threads, {dt:.1f} s", "single_image_s": t_one}
 
 
+def _dump_outputs(out_dir, **arrays):
+    """Writes each array as out_dir/<name>.npy in float32, so that two builds can be compared output for output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy().astype(np.float32))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -339,6 +347,7 @@ def run_ours(args):
     ev1.record()
     torch.cuda.synchronize()
     out = gathered if gathered is not None else last
+    dumped = out.cpu() if args.dump_outputs and rank == 0 else None   # before the extras below call the layer again
     if world > 1:
         dist.barrier()
     clocks = sampler.stop() if sampler is not None else None
@@ -561,6 +570,8 @@ def run_ours(args):
                 line["cpu_baseline"] = _cpu_baseline(mask, vertex, K, args.cpu_seconds)
             except Exception as e:   # the oracle is a checker; its absence must not hide the GPU number
                 line["cpu_baseline"] = {"value": None, "unit": UNIT, "cores": 0, "kind": "port", "sample": f"failed: {e}"}
+        if dumped is not None:
+            _dump_outputs(args.dump_outputs, keypoints=dumped)
         print(json.dumps(line))
         sys.stdout.flush()
     if world > 1:
@@ -674,7 +685,14 @@ def main():
                     help="profiling passes (ncu): timed steps only -- no extras, no end-to-end runs, no CPU baseline")
     ap.add_argument("--traffic", type=float, default=None,
                     help="dram bytes/launch of the vote kernel from the committed ncu capture (profiles/)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the keypoints [images of all ranks,K,2] of the last timed step to DIR/keypoints.npy (float32); the inputs "
+                         "and the step's seed depend only on the arguments, so two builds can be compared")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,4 +1,6 @@
 """Shared helpers for the GPU parity tests."""
+import hashlib
+
 import numpy as np
 import torch
 
@@ -22,6 +24,15 @@ def field_case(tn=2000, vn=3, hn=128, seed=0, noise_deg=3.0, outliers=0.2, exten
 
 def cuda(*arrays):
     return [torch.from_numpy(np.ascontiguousarray(a)).cuda() for a in arrays]
+
+
+def digest(*tensors):
+    """sha256 of the tensors' values in their logical (contiguous) order: pins inputs and byte-exact outputs that are
+    too large to store in tests/golden/."""
+    h = hashlib.sha256()
+    for t in tensors:
+        h.update(np.ascontiguousarray(t.detach().cpu().numpy()).tobytes())
+    return h.hexdigest()
 
 
 def bits_equal(a, b):
